@@ -43,6 +43,10 @@ def parse():
     p.add_argument("--cpu-baseline-seconds", type=float, default=12.0)
     p.add_argument("--no-cpu-baseline", action="store_true")
     p.add_argument("--pool", type=int, default=24, help="distinct resident input batches cycled through")
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps, write what the last one computed (loss; every parameter, its gradient and the "
+                        "floating-point buffers it updated) as DIR/<name>.npy; inputs and seeds are fixed by the arguments, "
+                        "so two builds can be compared output for output")
     return p.parse_args()
 
 
@@ -289,6 +293,34 @@ def time_second_variant(args, dev, precision, variant):
             "config": workload_config(a2, 1)["workload"]}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, loss, model):
+    """The step hands its caller the loss and updates the model in place: writes the loss, every parameter, its gradient
+    and the floating-point buffers (BatchNorm running statistics, quantizer ranges) as <out_dir>/<name>.npy."""
+    import numpy as np
+    arrays = {"loss": loss}
+    for name, p in model.named_parameters():
+        arrays[name] = p
+        if p.grad is not None:
+            arrays[name + ".grad"] = p.grad
+    for name, b in model.named_buffers():
+        if b.is_floating_point():
+            arrays[name] = b
+    host = {}
+    for name, t in arrays.items():
+        t = t.detach().cpu()
+        host[name] = (t if t.dtype in (torch.float32, torch.float64) else t.float()).numpy()
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    sys.stderr.write("[bench] wrote %d arrays (%d bytes) to %s\n" % (len(host), total, out_dir))
+
+
 def pick_precision(args, dev):
     """auto: the tcgen05 path (bf16 integer codes for q4, tf32 otherwise) if it passes a self-check, else fp32."""
     if args.precision != "auto":
@@ -421,6 +453,8 @@ def run_b200(args):
     ms = t_ms.item()
     value = world * B * args.steps / (ms * 1e-3)
     final_loss = loss_out.item()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loss_out, model)
 
     # ---------------- timed region 2: end to end through the public API with HOST buffers ("e2e")
     # Every step's input travels host (pinned) -> device inside the timed region; the copy of step i+1 is issued
@@ -556,10 +590,10 @@ def run_b200(args):
     lib_base = None
     if world == 1 and not args.no_library_baseline:
         try:
-            r = torch_gpu_arm(B, args.variant, 20, 5, dev)
+            r = torch_gpu_arm(B, args.variant, args.steps, args.warmup, dev)
             lib_base = {"value": r["img_s"], "unit": "img/s", "ms_per_step": r["ms_per_step"], "kind": "pytorch-eager",
-                        "sample": "20 steps of batch %d on the same GPU: the reference step (oracle port) in PyTorch eager -- "
-                                  "cuDNN / cuBLAS / ATen Philox, fp32" % B}
+                        "sample": "%d steps of batch %d on the same GPU: the reference step (oracle port) in PyTorch eager -- "
+                                  "cuDNN / cuBLAS / ATen Philox, fp32" % (args.steps, B)}
         except Exception as e:  # noqa: BLE001
             lib_base = {"unavailable": str(e)[:200]}
     h2d = B * 3 * 32 * 32 * 4 + B * 8

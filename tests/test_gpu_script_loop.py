@@ -2,22 +2,17 @@
 
 `tests/golden/script_trace.npz` holds the loss curve of the UNMODIFIED reference script (noisynet.py, q_a = q_w = 4,
 I = 1 nA, batch 64, --seed 0) over its first 60 steps on a deterministic synthetic dataset, minted in the build
-container by oracle/gen_script_trace.py.  The reference tree does not exist on the GPU box, so:
+container by oracle/gen_script_trace.py.
 
   * test_script_equivalent_loop_matches_reference_trace drives the drop-in modules (NoisyConv2d / NoisyLinear /
     QuantMeasure / add_noise_calculate_power in the script's two-call flow, the script's AdamW groups, per-step weight
     clamp, np.random permutation, `input.max()` live ranges of quantize2 / quantize4) through the SAME steps on the
     same data and compares the loss curve with the reference's own.  The generators differ (Philox streams of this
     library vs. ATen's), so the comparison is by windows: mean loss of steps 0-9, 25-34 and 50-59 within 0.12 of the
-    reference's, and the same downward trend;
-  * test_unmodified_script_on_gpu runs the real script under the drop-in modules when a reference tree IS present next
-    to a GPU (a maintainer's machine): same windows.
+    reference's, and the same downward trend.
 """
-import json
 import os
-import subprocess
 import sys
-import textwrap
 
 import numpy as np
 import pytest
@@ -26,7 +21,6 @@ import torch
 pytestmark = pytest.mark.gpu
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.environ.get("NOISYNET_REFERENCE", "/root/reference")
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
 
 
@@ -77,59 +71,3 @@ def test_script_equivalent_loop_matches_reference_trace(golden):
     assert ops.error_flag() == 0
     assert len(model.power[0]) == 20 and len(model.nsr[3]) == 20 and all(np.isfinite(model.power[1]))
     _check_against_trace(losses, trace)
-
-
-RUNNER = textwrap.dedent('''
-    import sys, types, runpy, collections.abc, json
-    import numpy as np, torch
-    sys.path.insert(0, {ref!r})
-    sys.path.insert(0, {dropin!r})
-    six = types.ModuleType('torch._six'); six.container_abcs = collections.abc
-    sys.modules['torch._six'] = six
-    mpl = types.ModuleType('matplotlib'); mpl.use = lambda *a, **k: None
-    plt = types.ModuleType('matplotlib.pyplot'); mpl.pyplot = plt
-    sys.modules['matplotlib'] = mpl; sys.modules['matplotlib.pyplot'] = plt
-    import hardware_model
-    assert 'noisynet_b200' in hardware_model.NoisyConv2d.__module__
-    np.random.seed(0)
-    losses = []
-    class Stop(Exception):
-        pass
-    _fwd = torch.nn.CrossEntropyLoss.forward
-    def fwd(self, out, lab):
-        l = _fwd(self, out, lab)
-        if torch.is_grad_enabled():
-            losses.append(float(l))
-        return l
-    torch.nn.CrossEntropyLoss.forward = fwd
-    _step = torch.optim.AdamW.step
-    count = [0]
-    def step(self, *a, **k):
-        r = _step(self, *a, **k)
-        count[0] += 1
-        if count[0] >= {steps}:
-            raise Stop()
-        return r
-    torch.optim.AdamW.step = step
-    sys.argv = ['noisynet.py'] + {argv!r}
-    try:
-        runpy.run_path({script!r}, run_name='__main__')
-    except Stop:
-        pass
-    json.dump(losses, open('losses.json', 'w'))
-''')
-
-
-@pytest.mark.skipif(not os.path.isfile(os.path.join(REF, "noisynet.py")), reason="reference tree not present on this machine")
-def test_unmodified_script_on_gpu(golden, tmp_path):
-    from gen_script_trace import synthetic_learnable_cifar
-    trace = golden("script_trace")
-    os.makedirs(tmp_path / "data")
-    x, y = synthetic_learnable_cifar(50000, seed=int(trace["data_seed"]))
-    xt, yt = synthetic_learnable_cifar(10000, seed=int(trace["data_seed"]) + 1)
-    np.savez(tmp_path / "data" / "cifar_RGB_4bit.npz", x, y, xt, yt)
-    code = RUNNER.format(ref=REF, dropin=os.path.join(ROOT, "dropin"), steps=int(trace["steps"]),
-                         argv=[str(v) for v in trace["argv"]], script=os.path.join(REF, "noisynet.py"))
-    r = subprocess.run([sys.executable, "-c", code], cwd=tmp_path, capture_output=True, text=True, timeout=1800)
-    assert os.path.isfile(tmp_path / "losses.json"), r.stdout[-1500:] + r.stderr[-3000:]
-    _check_against_trace(json.load(open(tmp_path / "losses.json")), trace)

@@ -1,7 +1,8 @@
 """Launch each hot contraction of the batch-512 step a few times (for ncu captures: conv1 forward / wgrad on the in-place
 kernels, conv2 forward / dgrad / wgrad on the TMA kernels)."""
+import os
 import sys
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 from noisynet_b200 import ops
 from noisynet_b200._lib import NOISE_EXTERNAL, NOISE_MERGED
